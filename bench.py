@@ -18,6 +18,13 @@ src/curve-random.ts:24-92), result returned to the host as the canonical affine 
           (weak scaling); each rank computes a partial sum, the partial accumulators are all-gathered
           with NCCL and every rank adds them and normalises (SURVEY.md 8e).
 
+--steps K sets the timed steps of every block of the line; the inputs depend only on the arguments.
+--dump-outputs DIR writes the result point of the last timed step of every timed loop as DIR/<name>.npy:
+float64 [x limbs, y limbs, isZero], x and y in little-endian 32-bit limbs (exact in float64).  Names:
+`msm` (scalars resident, the headline), `msm_e2e` (host scalars), `msm_e2e_pipelined` (host scalars,
+prefetched), the same three per `configs` entry and for `strong_2p24` (`<block>`, `<block>_e2e`, ...);
+the reference arm writes `msm`.  Two builds run with the same arguments can be compared file by file.
+
 The oracle (oracle/) is used here only for `cpu_baseline` and `--impl reference`.
 """
 import argparse
@@ -70,7 +77,25 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the `configs` / `strong_2p24` blocks (the other BASELINE configs)")
     ap.add_argument("--cpu-logn", type=int, default=0,
                     help="log2 size of the CPU baseline sample (0 = the whole workload when the host has >= 8 cores, else 2^18)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result point of the last timed step of every timed loop to DIR/<name>.npy (float64 32-bit limbs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+def result_limbs(res, coord_bytes):
+    """{x, y, isZero} -> float64 [x limbs, y limbs, isZero], x and y as little-endian 32-bit limbs."""
+    limbs = [(v >> (32 * i)) & 0xFFFFFFFF for v in (res["x"], res["y"]) for i in range(coord_bytes // 4)]
+    return np.array(limbs + [int(res["isZero"])], dtype=np.float64)
+
+
+def dump_outputs(out_dir, results):
+    """results: {name: (result point, coordinate bytes)} -> out_dir/<name>.npy"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (res, coord_bytes) in results.items():
+        np.save(os.path.join(out_dir, name + ".npy"), result_limbs(res, coord_bytes))
 
 
 class ClockSampler:
@@ -209,9 +234,11 @@ def run_reference(args):
     sets = [inputs.random_scalars(curve.q, n, SEED_SCALARS + i) for i in range(min(4, args.steps + args.warmup))]
     times = []
     for i in range(args.warmup + args.steps):
-        _, ms = cpu_reference_msm(args.curve, pts, sets[i % len(sets)], n, threads)
+        res, ms = cpu_reference_msm(args.curve, pts, sets[i % len(sets)], n, threads)
         if i >= args.warmup:
             times.append(ms)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"msm": (res, curve.coord_bytes)})
     ms_step = float(np.mean(times))
     value = n / (ms_step * 1e-3)
     sample = ("one MSM of 2^%d points per step (the whole per-GPU workload), %d threads" % (cl, threads)) if cl == args.logn else (
@@ -327,12 +354,22 @@ def run_b200(args):
         expect = O.result_of(O.scale(sum(ks) % O.q, O.G))
         parity_ok = bool(res == expect and res_e2e == expect and (res_pipe is None or res_pipe == expect))
         out = {"curve": curve, "n": n, "el": el, "el_e2e": el_e2e, "el_pipe": el_pipe, "phases_pipe": phases_pipe, "dev_ms_max": dev_ms_max, "phases": phases, "phases_e2e": phases_e2e,
-               "launches": launches, "res": res, "tm": tm, "clocks": clocks, "parity_ok": parity_ok, "sharded": sharded,
-               "host_sets": host_sets}
+               "launches": launches, "res": res, "res_e2e": res_e2e, "res_pipe": res_pipe, "tm": tm, "clocks": clocks, "parity_ok": parity_ok,
+               "sharded": sharded, "host_sets": host_sets}
         return out
+
+    outputs = {}        # --dump-outputs: the last timed step's result of every timed loop
+
+    def keep_outputs(block, r):
+        cb = r["curve"].coord_bytes
+        outputs[block] = (r["res"], cb)
+        outputs[block + "_e2e"] = (r["res_e2e"], cb)
+        if r["res_pipe"] is not None:
+            outputs[block + "_e2e_pipelined"] = (r["res_pipe"], cb)
 
     sampler = ClockSampler(local) if rank == 0 else None
     head = measure(args.curve, args.logn, SEED_POINTS, SEED_SCALARS, args.steps, args.warmup, sampler, c=args.c or None)
+    keep_outputs("msm", head)
     curve, n, phases, tm, sharded = head["curve"], head["n"], head["phases"], head["tm"], head["sharded"]
     eng = sharded.engine
     parity_ok = head["parity_ok"]
@@ -354,13 +391,14 @@ def run_b200(args):
 
     # ---- the other BASELINE configs (the named size on every GPU of the run, like the headline: weak scaling; the CPU port
     # beside them at N = 1) and config 5 (2^24 in total, every N)
-    extra_steps, extra_warm = max(3, min(args.steps, 10)), 3
+    extra_steps, extra_warm = args.steps, 3
     configs = {}
     cpu_host_threads = os.cpu_count() or 1
     if args.logn == LOGN_DEFAULT and args.curve == "bls12-377" and not args.no_extras:
         sharded.close()
         for name, cfg in EXTRA_CONFIGS.items():
             r = measure(cfg["curve"], cfg["logn"], SEED_POINTS ^ (cfg["seed_index"] + 1), 0x6D6F6E74 ^ cfg["seed_index"], extra_steps, extra_warm)
+            keep_outputs(name, r)
             nn = r["n"]
             dev_ms = r["dev_ms_max"]            # slowest rank (= this rank's phases["total"] at N = 1)
             where = "1 GPU" if world == 1 else "per GPU on %d GPUs (weak: %d x 2^%d pairs in total, one all-gather of the partial sums)" % (world, world, cfg["logn"])
@@ -389,8 +427,9 @@ def run_b200(args):
             sharded.close()
             head_engine_closed = True
         ln = STRONG_LOGN - (world.bit_length() - 1)
-        ssteps = max(2, min(args.steps, 5))
+        ssteps = args.steps
         r = measure("bls12-377", ln, SEED_POINTS ^ 0x5A5A, 0x6D6F6E74 ^ 4, ssteps, 2, nsets=2)
+        keep_outputs("strong_2p24", r)
         tot = (1 << ln) * world
         strong = {"workload": "bls12-377 G1 MSM, 2^%d points in total = 2^%d per GPU on %d GPU(s) (BASELINE config 5)" % (STRONG_LOGN, ln, world),
                   "scaling": "strong", "n_gpus": world, "ms_per_step": r["el"] / ssteps * 1e3, "ms_device_max": r["dev_ms_max"],
@@ -475,6 +514,8 @@ def run_b200(args):
                                            "one MSM of the first 2^%d points of the workload, %.0f ms") % (cl, cms),
                                 "agrees_with_gpu": cres == gres}
         ceng.close()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     sys.stdout.flush()
     os.dup2(saved_fd, 1)
     os.close(saved_fd)
@@ -486,6 +527,7 @@ def run_b200(args):
 
 
 def main():
+    sys.dont_write_bytecode = True      # the tree bench.py runs from may be read-only: no bytecode caches in it
     args = parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -64,3 +64,13 @@ def points_to_bytes(points, coord_bytes):
 
 def scalars_to_bytes(scalars):
     return np.frombuffer(b"".join(int(s).to_bytes(32, "little") for s in scalars), dtype=np.uint8).reshape(-1, 32).copy()
+
+
+def dumped_point(path, coord_bytes):
+    """A result point written by `bench.py --dump-outputs` (float64 [x limbs, y limbs, isZero], 32-bit limbs) -> result dict."""
+    v = np.load(path)
+    nl = coord_bytes // 4
+    assert v.dtype == np.float64 and v.shape == (2 * nl + 1,)
+    assert all(0 <= w < 2**32 and w == int(w) for w in v[:-1]) and v[-1] in (0, 1)
+    x, y = (sum(int(w) << (32 * i) for i, w in enumerate(v[k * nl:(k + 1) * nl])) for k in (0, 1))
+    return {"x": x, "y": y, "isZero": bool(v[-1])}

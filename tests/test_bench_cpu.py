@@ -38,6 +38,20 @@ def test_reference_arm_prints_the_contract_line():
     assert line["gpu_launches"] == 0 and line["vs_baseline"] is None
 
 
+def test_reference_arm_dumps_the_last_step(tmp_path):
+    """--dump-outputs: the result of the last timed step (set (warmup + steps - 1) mod 3 of the seeded scalar sets against
+    the seeded known-dlog points), which must be the closed form of those inputs"""
+    from montgomery_b200 import inputs
+    from tests.helpers import OracleCurve, dumped_point
+    res = _run(None, "--dump-outputs", str(tmp_path / "out"))
+    assert res.returncode == 0, res.stderr[-2000:]
+    assert os.listdir(tmp_path / "out") == ["msm.npy"]
+    O = OracleCurve("bls12-377")
+    n = 1 << 11
+    k = inputs.dot_known_dlogs(inputs.random_scalars(O.q, n, bench.SEED_SCALARS + 2), inputs.known_dlogs(bench.SEED_POINTS, n))
+    assert dumped_point(tmp_path / "out" / "msm.npy", 48) == O.result_of(O.scale(k % O.q, O.G))
+
+
 def test_reference_arm_under_a_multi_rank_launch():
     """torchrun starts one process per GPU; rank 0 alone runs and prints, the others exit 0 without work"""
     quiet = _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}, "--gpus", "2")
