@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmontgomery_b200.so")
 OBJDIR = os.path.join(HERE, "build")
 SOURCES = ["msm.cu", "tools.cu"]
-HEADERS = ["ptx.cuh", "field.cuh", "ec.cuh", "coop.cuh", "warp.cuh", "engine.cuh", "constants_gen.cuh", os.path.join("..", "..", "include", "montgomery_b200.h")]
+HEADERS = ["ptx.cuh", "field.cuh", "ec.cuh", "coop.cuh", "warp.cuh", "onewarp.cuh", "engine.cuh", "constants_gen.cuh", os.path.join("..", "..", "include", "montgomery_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
     "-Xcompiler", "-fPIC", "-Xptxas", "-v",

@@ -1,4 +1,9 @@
 """Shared test helpers: oracle curve objects and conversions (tests may import oracle/)."""
+import glob
+import hashlib
+import os
+import subprocess
+
 import numpy as np
 
 from oracle.params import BLS12_377, BLS12_381, ED_ON_BLS12_377, PALLAS
@@ -6,6 +11,7 @@ from oracle.twisted_edwards import TwistedEdwardsCurve
 from oracle.weierstrass import AffineCurve, ProjectiveCurve
 from oracle.msm import msm as oracle_msm
 
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_PARAMS = {"bls12-377": BLS12_377, "pallas": PALLAS, "ed-on-bls12-377": ED_ON_BLS12_377, "bls12-381": BLS12_381}
 
 
@@ -64,6 +70,38 @@ def points_to_bytes(points, coord_bytes):
 
 def scalars_to_bytes(scalars):
     return np.frombuffer(b"".join(int(s).to_bytes(32, "little") for s in scalars), dtype=np.uint8).reshape(-1, 32).copy()
+
+
+GPU_UNITS_SRC = os.path.join(ROOT, "tests", "gpu_units", "units.cu")
+
+
+def gpu_units_flags():
+    """The product library's code generation (montgomery_b200.build.NVCC_FLAGS + MGB_NVCC_EXTRA)."""
+    from montgomery_b200 import build as b
+    return b.NVCC_FLAGS + os.environ.get("MGB_NVCC_EXTRA", "").split()
+
+
+def gpu_units_key():
+    """Hash of the test harness tests/gpu_units/units.cu, every file of csrc/, the public header and the flags."""
+    from montgomery_b200 import build as b
+    h = hashlib.sha256()
+    files = [GPU_UNITS_SRC] + sorted(glob.glob(os.path.join(b.CSRC, "*"))) + [os.path.join(ROOT, "include", "montgomery_b200.h")]
+    for f in files:
+        h.update(os.path.basename(f).encode() + b"\0")
+        with open(f, "rb") as fh:
+            h.update(fh.read())
+    h.update(" ".join(gpu_units_flags()).encode())
+    return h.hexdigest()[:20]
+
+
+def compile_gpu_units(so_path):
+    """nvcc tests/gpu_units/units.cu -> so_path (sm_100a, the product's flags); returns the compiler output."""
+    from montgomery_b200 import build as b
+    cmd = [b._nvcc()] + gpu_units_flags() + ["-shared", "-o", so_path, GPU_UNITS_SRC, "-lcudart"]
+    res = subprocess.run(cmd, capture_output=True, text=True)
+    if res.returncode != 0:
+        raise RuntimeError("nvcc failed for tests/gpu_units/units.cu:\n" + (res.stdout + res.stderr)[-4000:])
+    return res.stdout + res.stderr
 
 
 def dumped_point(path, coord_bytes):
