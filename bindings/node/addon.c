@@ -7,7 +7,9 @@
  *
  * Exports (all take the context handle returned by create):
  *   create(curve, device, maxPoints) -> External            mgb_create        (Weierstrass.create + startThreads)
- *   setPoints(ctx, Uint8Array xy, n)                         mgb_set_points    (Parallel.pointsFromBytes)
+ *   setPoints(ctx, Uint8Array xy, n[, check])                mgb_set_points    (Parallel.pointsFromBytes); check = 1:
+ *                                                            mgb_set_points_checked (isOnCurve / isInSubgroup of every
+ *                                                            point on the GPU), throws its message on an invalid point
  *   randomPoints(ctx, seed, n)                               mgb_random_points (Parallel.randomPointsFast)
  *   msm(ctx, Uint8Array scalars, n, c, projective) -> Promise<{xy: Uint8Array, isZero, log}>
  *                                                            mgb_msm on a libuv worker thread, so the event loop is
@@ -45,8 +47,9 @@ static napi_value Create(napi_env env, napi_callback_info info) {
 }
 
 static napi_value SetPoints(napi_env env, napi_callback_info info) {
-  size_t argc = 3, len; napi_value argv[3]; void* data; int64_t n; napi_typedarray_type ty; mgb_ctx* ctx;
+  size_t argc = 4, len; napi_value argv[4]; void* data; int64_t n; int32_t check = 0; napi_typedarray_type ty; mgb_ctx* ctx;
   CHECK(napi_get_cb_info(env, info, &argc, argv, NULL, NULL));
+  if (argc >= 4) CHECK(napi_get_value_int32(env, argv[3], &check));
   if (!(ctx = ctx_of(env, argv[0]))) return NULL;
   CHECK(napi_get_typedarray_info(env, argv[1], &ty, &len, &data, NULL, NULL));
   CHECK(napi_get_value_int64(env, argv[2], &n));
@@ -55,7 +58,9 @@ static napi_value SetPoints(napi_env env, napi_callback_info info) {
     napi_throw_range_error(env, NULL, "points: the buffer must hold exactly n points of 2 * 32 or 2 * 48 bytes");   /* never read past the array */
     return NULL;
   }
-  if (mgb_set_points(ctx, (const uint8_t*)data, NULL, (size_t)n) != MGB_OK) napi_throw_error(env, NULL, mgb_last_error(ctx));
+  if ((check ? mgb_set_points_checked(ctx, (const uint8_t*)data, NULL, (size_t)n, NULL, NULL)
+             : mgb_set_points(ctx, (const uint8_t*)data, NULL, (size_t)n)) != MGB_OK)
+    napi_throw_error(env, NULL, mgb_last_error(ctx));
   return NULL;
 }
 

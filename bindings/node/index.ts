@@ -26,9 +26,12 @@ export function create(curve: Curve, { device = 0, maxPoints = 1 << 20 } = {}) {
     return { result: { x: fromLE(xy.subarray(0, cb)), y: fromLE(xy.subarray(cb, 2 * cb)), isZero }, log };
   }
   const Parallel = {
-    pointsFromBytes(bytes: Uint8Array): Points {                // src/parallel.ts:97-116 / :209-232
+    // src/parallel.ts:97-116 / :209-232.  check: every point is checked on the GPU (canonical, on the curve, in the
+    // prime-order subgroup: isOnCurve / isInSubgroup); an invalid one throws "<count> invalid points; the first is point
+    // <i>: <reason>" and the engine holds no points.
+    pointsFromBytes(bytes: Uint8Array, { check = false } = {}): Points {
       const n = bytes.length / (2 * cb);
-      addon.setPoints(ctx, bytes, n);
+      addon.setPoints(ctx, bytes, n, check ? 1 : 0);
       return { n };
     },
     randomPointsFast(n: number, seed = 0x6d6f6e74): Points {    // src/curve-random.ts:24-92

@@ -92,6 +92,25 @@ int mgb_create(mgb_ctx** out, int curve, int device, size_t max_points);
  * as the neutral element (the reference's `isNonZero` flag, src/curve-affine.ts:20-52). */
 int mgb_set_points(mgb_ctx* ctx, const uint8_t* xy_le, const uint8_t* is_zero, size_t n);
 
+/* mgb_set_points for points from outside (SRS files, another library's output, bytes off the wire): the same
+ * ingestion, and every point is checked on the device as it is ingested -- the reference's `isOnCurve` and
+ * `isInSubgroup` of its curve types (src/curve-projective.ts, src/curve-twisted-edwards.ts), one thread per point.
+ * Each point gets a status byte, a mask of the MGB_PT_* bits below (0 = valid; a point flagged in is_zero is valid
+ * whatever its coordinate bytes are).  A non-canonical encoding gets MGB_PT_NONCANONICAL alone; the curve equation is
+ * checked on canonical points, and MGB_PT_NOT_IN_SUBGROUP is set only for points on the curve.  Subgroup tests:
+ * Pallas has cofactor 1; BLS12-377 / BLS12-381 G1 test sigma'(P) + P == [z^2] P with the endomorphism of eigenvalue
+ * z^2 - 1 (exact, DESIGN.md "Checked point ingestion"); ed-on-BLS12-377 tests [q] P == O.
+ * All points valid: returns MGB_OK and stores the table mgb_set_points would store from the same bytes.
+ * Any point invalid: returns MGB_E_INVALID, mgb_last_error names the count and the first invalid index with its reason,
+ * and the context holds NO points afterwards (mgb_msm returns MGB_E_STATE, as on a fresh context).
+ * `status` (n bytes) and `n_invalid` may be NULL; the count and the first index are kept on the device either way.
+ * Device memory: one byte per point plus 8 bytes, allocated by the first call and kept by the context. */
+#define MGB_PT_NONCANONICAL 1      /* x or y >= p (from the raw bytes)                                       */
+#define MGB_PT_OFF_CURVE 2         /* the point does not satisfy the curve equation                          */
+#define MGB_PT_NOT_IN_SUBGROUP 4   /* on the curve, not in the prime-order subgroup                          */
+int mgb_set_points_checked(mgb_ctx* ctx, const uint8_t* xy_le, const uint8_t* is_zero, size_t n,
+                           uint8_t* status /* n bytes, may be NULL */, uint64_t* n_invalid /* may be NULL */);
+
 /* Replaces `Parallel.randomPointsFast(n)` (src/curve-random.ts:24-92): fills the context with n
  * points a_i*G, a_i a seeded 64-bit value (splitmix64 of seed and i), built on the device from
  * a 64-step double-and-add of the generator, one thread per point.  Deterministic; used for benchmarks
@@ -178,6 +197,11 @@ int mgb_msm_sharded(mgb_ctx* ctx, const void* scalars, int scalars_on_device, si
 typedef struct mgb_multi mgb_multi;
 int mgb_multi_create(mgb_multi** out, int curve, const int* device_ids, int n_devices, size_t max_points_per_device);
 int mgb_multi_set_points(mgb_multi* m, const uint8_t* xy_le, const uint8_t* is_zero, size_t n);
+/* mgb_set_points_checked over the shards (isOnCurve / isInSubgroup of the reference): every device checks its shard at
+ * the same time; status, the count and the first index in the message are global.  If any shard holds an invalid point,
+ * returns MGB_E_INVALID and EVERY device is left without points. */
+int mgb_multi_set_points_checked(mgb_multi* m, const uint8_t* xy_le, const uint8_t* is_zero, size_t n,
+                                 uint8_t* status /* n bytes, may be NULL */, uint64_t* n_invalid /* may be NULL */);
 int mgb_multi_random_points(mgb_multi* m, uint64_t seed, size_t n);
 int mgb_multi_get_points(mgb_multi* m, size_t first, size_t n, uint8_t* xy_le, uint8_t* is_zero);
 int mgb_multi_msm(mgb_multi* m, const uint8_t* scalars_le32, size_t n, const mgb_opts* opts,

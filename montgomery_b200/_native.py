@@ -31,15 +31,16 @@ class MgbTiming(ctypes.Structure):
 
 
 EXPORTS = [
-    "mgb_create", "mgb_set_points", "mgb_random_points", "mgb_get_points", "mgb_msm", "mgb_msm_prefetch", "mgb_msm_device",
+    "mgb_create", "mgb_set_points", "mgb_set_points_checked", "mgb_random_points", "mgb_get_points", "mgb_msm", "mgb_msm_prefetch", "mgb_msm_device",
     "mgb_partial_bytes", "mgb_msm_partial", "mgb_combine_partials", "mgb_field_op", "mgb_microbench",
     "mgb_last_error", "mgb_destroy",
     "mgb_comm_unique_id", "mgb_comm_init", "mgb_comm_info", "mgb_msm_sharded",
-    "mgb_multi_create", "mgb_multi_set_points", "mgb_multi_random_points", "mgb_multi_get_points", "mgb_multi_msm",
+    "mgb_multi_create", "mgb_multi_set_points", "mgb_multi_set_points_checked", "mgb_multi_random_points", "mgb_multi_get_points", "mgb_multi_msm",
     "mgb_multi_last_error", "mgb_multi_destroy",
 ]
 COMM_ID_BYTES = 128
 E_INVALID, E_CUDA, E_NOMEM, E_STATE, E_COMM = -1, -2, -3, -4, -5
+PT_NONCANONICAL, PT_OFF_CURVE, PT_NOT_IN_SUBGROUP = 1, 2, 4      # status bits of mgb_set_points_checked
 
 
 def load():
@@ -51,6 +52,7 @@ def load():
     vp, sz, ci = ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int
     lib.mgb_create.argtypes = [ctypes.POINTER(vp), ci, ci, sz]
     lib.mgb_set_points.argtypes = [vp, vp, vp, sz]
+    lib.mgb_set_points_checked.argtypes = [vp, vp, vp, sz, vp, ctypes.POINTER(ctypes.c_uint64)]
     lib.mgb_random_points.argtypes = [vp, ctypes.c_uint64, sz]
     lib.mgb_get_points.argtypes = [vp, sz, sz, vp, vp]
     lib.mgb_msm.argtypes = [vp, vp, sz, ctypes.POINTER(MgbOpts), vp, ctypes.POINTER(ci), ctypes.POINTER(MgbTiming)]
@@ -73,6 +75,7 @@ def load():
     lib.mgb_msm_sharded.argtypes = [vp, vp, ci, sz, ctypes.POINTER(MgbOpts), vp, pi, ctypes.POINTER(MgbTiming)]
     lib.mgb_multi_create.argtypes = [ctypes.POINTER(vp), ci, pi, ci, sz]
     lib.mgb_multi_set_points.argtypes = [vp, vp, vp, sz]
+    lib.mgb_multi_set_points_checked.argtypes = [vp, vp, vp, sz, vp, ctypes.POINTER(ctypes.c_uint64)]
     lib.mgb_multi_random_points.argtypes = [vp, ctypes.c_uint64, sz]
     lib.mgb_multi_get_points.argtypes = [vp, sz, sz, vp, vp]
     lib.mgb_multi_msm.argtypes = [vp, vp, sz, ctypes.POINTER(MgbOpts), vp, pi, ctypes.POINTER(MgbTiming)]

@@ -24,6 +24,32 @@ class MsmError(RuntimeError):
         self.code = code
 
 
+# status bits of a point checked on ingestion (set_points(..., check=True)); 0 = valid
+PT_NONCANONICAL = _native.PT_NONCANONICAL          # x or y >= p
+PT_OFF_CURVE = _native.PT_OFF_CURVE                # not on the curve
+PT_NOT_IN_SUBGROUP = _native.PT_NOT_IN_SUBGROUP    # on the curve, not in the prime-order subgroup
+
+
+class InvalidPointsError(MsmError):
+    """set_points(..., check=True) found invalid points; the engine then holds no points.  `status` is the per-point
+    np.uint8 array of PT_* bits, `count` the number of invalid points, `first` the index of the first one."""
+
+    def __init__(self, code, msg, status, count, first):
+        super().__init__(code, msg)
+        self.status, self.count, self.first = status, count, first
+
+
+def _set_points_checked(fn, handle, xy, zp, n, error_of):
+    """mgb_set_points_checked / mgb_multi_set_points_checked -> None, or raises InvalidPointsError / MsmError"""
+    status = np.zeros(n, dtype=np.uint8)
+    count = ctypes.c_uint64(0)
+    rc = fn(handle, _ptr(xy), zp, n, _ptr(status), ctypes.byref(count))
+    if rc == _native.E_INVALID and count.value:
+        raise InvalidPointsError(rc, error_of(), status, int(count.value), int(np.flatnonzero(status)[0]))
+    if rc != 0:
+        raise MsmError(rc, error_of())
+
+
 def _ptr(a: np.ndarray):
     return a.ctypes.data_as(ctypes.c_void_p)
 
@@ -68,7 +94,9 @@ class MsmEngine:
             pass
 
     # ---- points
-    def set_points(self, xy_bytes, is_zero=None):
+    def set_points(self, xy_bytes, is_zero=None, check=False):
+        """check=True: mgb_set_points_checked -- every point is checked on the device (canonical encoding, on the curve,
+        in the prime-order subgroup); an invalid one raises InvalidPointsError and leaves the engine without points."""
         xy = np.ascontiguousarray(np.frombuffer(xy_bytes, dtype=np.uint8) if not isinstance(xy_bytes, np.ndarray) else xy_bytes.reshape(-1))
         pb = self.curve.point_bytes
         if xy.size % pb:
@@ -79,7 +107,11 @@ class MsmEngine:
             z = np.ascontiguousarray(np.asarray(is_zero, dtype=np.uint8))
             assert z.size == n
             zp = _ptr(z)
-        self._check(self.lib.mgb_set_points(self._h, _ptr(xy), zp, n))
+        if check:
+            self.n_points = 0
+            _set_points_checked(self.lib.mgb_set_points_checked, self._h, xy, zp, n, lambda: self.lib.mgb_last_error(self._h).decode())
+        else:
+            self._check(self.lib.mgb_set_points(self._h, _ptr(xy), zp, n))
         self.n_points = n
         return n
 
@@ -209,11 +241,17 @@ class MultiGpuMsm:
         if rc != 0:
             raise MsmError(rc, self.lib.mgb_multi_last_error(self._h).decode())
 
-    def set_points(self, xy_bytes, is_zero=None):
+    def set_points(self, xy_bytes, is_zero=None, check=False):
+        """check=True: mgb_multi_set_points_checked (see MsmEngine.set_points); status and `first` are global indices,
+        and an invalid point in any shard leaves every device without points."""
         xy = np.ascontiguousarray(np.frombuffer(xy_bytes, dtype=np.uint8) if not isinstance(xy_bytes, np.ndarray) else xy_bytes.reshape(-1))
         n = xy.size // self.curve.point_bytes
         z = None if is_zero is None else np.ascontiguousarray(np.asarray(is_zero, dtype=np.uint8))
-        self._check(self.lib.mgb_multi_set_points(self._h, _ptr(xy), None if z is None else _ptr(z), n))
+        zp = None if z is None else _ptr(z)
+        if check:
+            _set_points_checked(self.lib.mgb_multi_set_points_checked, self._h, xy, zp, n, lambda: self.lib.mgb_multi_last_error(self._h).decode())
+        else:
+            self._check(self.lib.mgb_multi_set_points(self._h, _ptr(xy), zp, n))
         return n
 
     def random_points(self, n, seed):
@@ -277,10 +315,16 @@ class _Parallel:
         self._m._owner = weakref.ref(ps)
         return ps
 
-    def pointsFromBytes(self, point_bytes, is_zero=None):
+    def pointsFromBytes(self, point_bytes, is_zero=None, check=False):
+        """check=True: the points are checked on the device as they are ingested (the reference's isOnCurve /
+        isInSubgroup); an invalid point raises InvalidPointsError and no PointSet is returned."""
         n = len(point_bytes) // self._m.curve.point_bytes
         ps = self._new_point_set(n)
-        ps.engine.set_points(point_bytes, is_zero)
+        try:
+            ps.engine.set_points(point_bytes, is_zero, check=check)
+        except MsmError:
+            ps.close()
+            raise
         return ps
 
     def scalarsFromBytes(self, scalar_bytes):

@@ -60,6 +60,11 @@ static constexpr uint32_t REF_ENDO = 0x40000000u;
 static constexpr uint32_t REF_IDX = 0x3fffffffu;
 static constexpr uint32_t NO_BUCKET = 0xffffffffu;
 
+// status bits of a point checked on ingestion (MGB_PT_* of include/montgomery_b200.h)
+static constexpr uint32_t PT_NONCANONICAL = 1;
+static constexpr uint32_t PT_OFF_CURVE = 2;
+static constexpr uint32_t PT_NOT_IN_SUBGROUP = 4;
+
 // ---------------------------------------------------------------- curve policies
 template <class FP, class CC, class GL, int MAGB>
 struct WeierstrassPolicy {
@@ -167,6 +172,35 @@ struct WeierstrassPolicy {
     const Fe<FP> izz = F::mul(F::sqr(t), F::sqr(a.ZZ));
     x = F::from_mont(F::mul(a.X, izz)); y = F::from_mont(F::mul(a.Y, t));
   }
+  // Status bits (PT_*) of a table entry made from canonical coordinates: the curve equation 3(y^2 - x^3) == 3b, then
+  // membership of the prime-order subgroup.  BLS12: sigma'(P) == [z^2 - 1] P (sigma' has the eigenvalue z^2 - 1 on G1;
+  // DESIGN.md "Checked point ingestion" proves the test exact).  [z^2] P is one fixed double-and-add chain over the
+  // 127/128-bit z^2 with mixed additions of the affine P, which is re-read from the table: one XYZZ accumulator is all
+  // that lives across the chain (two chains over |z| would keep a second one and spill at 3 blocks per SM).  The chain
+  // is a compile-time constant, so every lane of a warp runs the same instructions; the complete formulas branch only
+  // on adversarial points.
+  MGB_DEV static uint32_t check_entry(const uint32_t* e) {
+    vpoint p = load_entry(e, 0, false, false);
+    if (G::is_inf(p)) return 0;
+    Fe<FP> b3; _Pragma("unroll") for (int i = 0; i < N; i++) b3.v[i] = CC::b3(i);
+    const Fe<FP> t = F::sub(F::sqr(p.y), F::mul(F::sqr(p.x), p.x));
+    if (!F::eq(F::add(F::dbl(t), t), b3)) return PT_OFF_CURVE;
+    if (CC::Z2_TOP < 0) return 0;                                   // cofactor 1
+    acc a = G::from_affine(p);                                      // the top bit of z^2
+    _Pragma("unroll") for (int half = 1; half >= 0; half--) {
+      const uint64_t word = half ? CC::Z2_HI : CC::Z2_LO;
+      _Pragma("unroll 1") for (int bit = (half ? CC::Z2_TOP - 64 : 64) - 1; bit >= 0; bit--) {
+        a = G::dbl(a);
+        if ((word >> bit) & 1) a = G::madd(a, load_entry(e, 0, false, false));
+      }
+    }
+    a = G::madd(a, load_entry(e, 0, false, true));                  // [z^2 - 1] P
+    vpoint s = load_entry(e, 0, true, false);                       // sigma'(P) = (beta x, y) or (beta^2 x, y)
+    if (CC::SIGMA_BETA_SQUARED) { Fe<FP> beta; _Pragma("unroll") for (int i = 0; i < N; i++) beta.v[i] = CC::beta(i); s.x = F::mul(s.x, beta); }
+    // sigma'(P) (affine, never infinity) == [z^2 - 1] P (XYZZ) without inversion: x ZZ == X and y ZZZ == Y
+    const bool same = !G::acc_is_zero(a) && F::eq(F::mul(s.x, a.ZZ), a.X) && F::eq(F::mul(s.y, a.ZZZ), a.Y);
+    return same ? 0 : PT_NOT_IN_SUBGROUP;
+  }
 };
 
 template <class FP, class CC>
@@ -261,6 +295,25 @@ struct TwistedEdwardsPolicy {
     x = F::from_mont(F::mul(a.X, zi)); y = F::from_mont(F::mul(a.Y, zi));
     Fe<FP> o = F::zero(); o.v[0] = 1;
     inf = F::is_zero(x) && F::eq(y, o);
+  }
+  // Status bits (PT_*) of a table entry made from canonical coordinates: -x^2 + y^2 = 1 + d x^2 y^2, i.e.
+  // 2(y^2 - x^2 - 1) == k x^2 y^2, then [q]P == O by the fixed signed-digit chain of q (constants_gen.cuh: 250
+  // doublings, 87 mixed additions of +-P).  The neutral element (the entry of a point flagged as zero) passes both.
+  MGB_DEV static uint32_t check_entry(const uint32_t* e) {
+    typename G::affine p; p.x = ld_fe<FP>(e); p.y = ld_fe<FP>(e + N); p.kt = ld_fe<FP>(e + 3 * N);
+    const Fe<FP> xx = F::sqr(p.x), yy = F::sqr(p.y);
+    if (!F::eq(F::dbl(F::sub(F::sub(yy, xx), F::one())), F::mul(F::mul(xx, yy), G::k2d()))) return PT_OFF_CURVE;
+    const typename G::affine np = G::neg(p);
+    acc r = G::from_affine(p);                                      // the top digit is +1
+    _Pragma("unroll") for (int w = CC::NAF_TOP / 32; w >= 0; w--) {
+      const uint32_t pos = CC::naf_pos(w), neg = CC::naf_neg(w);
+      _Pragma("unroll 1") for (int bit = (w == CC::NAF_TOP / 32 ? CC::NAF_TOP % 32 : 32) - 1; bit >= 0; bit--) {
+        r = G::dbl(r);
+        if ((pos >> bit) & 1) r = G::madd(r, p);
+        if ((neg >> bit) & 1) r = G::madd(r, np);
+      }
+    }
+    return F::is_zero(r.X) && !F::is_zero(r.Z) && F::eq(r.Y, r.Z) ? 0 : PT_NOT_IN_SUBGROUP;
   }
 };
 
@@ -1391,12 +1444,42 @@ __global__ void __launch_bounds__(32) k_normalize(const uint32_t* __restrict__ a
 }
 
 // ---------------------------------------------------------------- point ingestion / generation
-template <class CV>
-__global__ void __launch_bounds__(128) k_set_points(uint32_t n, const uint32_t* __restrict__ xy, const uint8_t* __restrict__ is_zero, uint32_t* __restrict__ table) {
+template <class FP>
+MGB_DEV bool below_modulus(const Fe<FP>& a) {   // a < p, on the raw limbs
+  uint32_t borrow = 0;
+  _Pragma("unroll") for (int i = 0; i < FP::N; i++) borrow = (uint32_t)(((uint64_t)a.v[i] - FP::mod(i) - borrow) >> 32) & 1u;
+  return borrow != 0;
+}
+// CHECK (mgb_set_points_checked): also status[i] = PT_NONCANONICAL when x or y >= p, else 0 -- k_check_points then adds
+// the curve and subgroup bits.  A point flagged as zero is valid whatever its coordinate bytes are.
+template <class CV, bool CHECK = false>
+__global__ void __launch_bounds__(128) k_set_points(uint32_t n, const uint32_t* __restrict__ xy, const uint8_t* __restrict__ is_zero, uint32_t* __restrict__ table,
+                                                    uint8_t* __restrict__ status = nullptr) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   Fe<typename CV::P> x = ld_fe<typename CV::P>(xy + (size_t)i * 2 * CV::N), y = ld_fe<typename CV::P>(xy + (size_t)i * 2 * CV::N + CV::N);
-  CV::make_entry(table + (size_t)i * CV::ENTRY_LIMBS, x, y, is_zero ? is_zero[i] != 0 : false);
+  const bool inf = is_zero ? is_zero[i] != 0 : false;
+  CV::make_entry(table + (size_t)i * CV::ENTRY_LIMBS, x, y, inf);
+  if (CHECK) status[i] = inf || (below_modulus(x) && below_modulus(y)) ? 0 : (uint8_t)PT_NONCANONICAL;
+}
+// The curve and subgroup checks of mgb_set_points_checked over the resident table, one thread per point.  A point that
+// k_set_points<CV, true> found non-canonical keeps that bit alone (its entry holds the coordinates mod p, not the input).
+// counters[0] += number of invalid points; counters[1] = max(counters[1], ~index): the largest complement is that of
+// the first invalid index (0: none).  The minimum of three blocks per SM keeps 12 warps resident (3 per scheduler):
+// the chains are throughput-bound products (DESIGN.md §3).
+template <class CV>
+__global__ void __launch_bounds__(128, 3) k_check_points(uint32_t n, const uint32_t* __restrict__ table, uint8_t* __restrict__ status, uint32_t* __restrict__ counters) {
+  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  uint32_t s = status[i];
+  if (s == 0) {
+    s = CV::check_entry(table + (size_t)i * CV::ENTRY_LIMBS);
+    status[i] = (uint8_t)s;
+  }
+  if (s) {
+    atomicAdd(&counters[0], 1u);
+    atomicMax(&counters[1], ~i);
+  }
 }
 template <class CV>
 __global__ void __launch_bounds__(128) k_get_points(uint32_t first, uint32_t n, const uint32_t* __restrict__ table, uint32_t* __restrict__ xy, uint8_t* __restrict__ is_zero) {

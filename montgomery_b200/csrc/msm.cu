@@ -43,6 +43,7 @@ struct mgb_ctx {
   cudaEvent_t ev_fork = nullptr, ev_plan = nullptr, ev_join[3] = {}, ev_chunk[4] = {};
   cudaEvent_t ev[EV_COUNT] = {};
   DevBuf table, scalars, ent_bucket, ent_rank, counts, offs, offcnt, tile_sums, pairs, pairs2, V, W, recs, lifes, prebuf, bsum, redU[2], redW[2], misc, acc_out, out_xy, stage;
+  DevBuf checks;                 // mgb_set_points_checked only: two counters, then one status byte per point
   uint32_t* h_pinned = nullptr;  // [0..31] out xy limbs + flag, [64..] misc readback
   int sm_count = 148;
   std::string err;
@@ -169,8 +170,9 @@ inline unsigned cdiv(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
 // copies).  Large point sets travel in chunks through two staging halves: the copy of chunk k + 1 runs on the copy
 // stream while k_set_points converts chunk k, and the staging memory stays bounded (2 x 2^18 points) instead of a second
 // copy of the whole input.  Small sets are one copy and one launch.
+// d_status (checked ingestion): k_set_points also writes the canonical-encoding bit of each point there.
 template <class CV>
-int set_points_impl(mgb_ctx* ctx, const uint8_t* xy, const uint8_t* is_zero, size_t n) {
+int set_points_impl(mgb_ctx* ctx, const uint8_t* xy, const uint8_t* is_zero, size_t n, uint8_t* d_status = nullptr) {
   const size_t pbytes = 2 * CV::COORD_BYTES;
   size_t chunk = (size_t)1 << 18;
   if (const char* ev = getenv("MGB_DEBUG_INGEST_CHUNK")) chunk = std::max(1, atoi(ev));   // (tests: several chunks of a small set)
@@ -183,7 +185,8 @@ int set_points_impl(mgb_ctx* ctx, const uint8_t* xy, const uint8_t* is_zero, siz
       dz = (uint8_t*)ctx->stage.p + n * pbytes;
       CU(ctx, cudaMemcpyAsync(dz, is_zero, n, cudaMemcpyHostToDevice, ctx->stream));
     }
-    k_set_points<CV><<<cdiv(n, 128), 128, 0, ctx->stream>>>((uint32_t)n, (const uint32_t*)ctx->stage.p, dz, table);
+    if (d_status) k_set_points<CV, true><<<cdiv(n, 128), 128, 0, ctx->stream>>>((uint32_t)n, (const uint32_t*)ctx->stage.p, dz, table, d_status);
+    else k_set_points<CV><<<cdiv(n, 128), 128, 0, ctx->stream>>>((uint32_t)n, (const uint32_t*)ctx->stage.p, dz, table);
     CU(ctx, cudaGetLastError());
   } else {
     const size_t half = (chunk * (pbytes + 1) + 255) / 256 * 256;     // one staging half: the chunk's x||y bytes, then its flags
@@ -205,13 +208,45 @@ int set_points_impl(mgb_ctx* ctx, const uint8_t* xy, const uint8_t* is_zero, siz
       }
       CU(ctx, cudaEventRecord(landed[h], cs));
       CU(ctx, cudaStreamWaitEvent(ctx->stream, landed[h], 0));
-      k_set_points<CV><<<cdiv(cnt, 128), 128, 0, ctx->stream>>>((uint32_t)cnt, (const uint32_t*)sp, dz, table + b * CV::ENTRY_LIMBS);
+      if (d_status) k_set_points<CV, true><<<cdiv(cnt, 128), 128, 0, ctx->stream>>>((uint32_t)cnt, (const uint32_t*)sp, dz, table + b * CV::ENTRY_LIMBS, d_status + b);
+      else k_set_points<CV><<<cdiv(cnt, 128), 128, 0, ctx->stream>>>((uint32_t)cnt, (const uint32_t*)sp, dz, table + b * CV::ENTRY_LIMBS);
       CU(ctx, cudaGetLastError());
       CU(ctx, cudaEventRecord(drained[h], ctx->stream));
     }
   }
   CU(ctx, cudaStreamSynchronize(ctx->stream));
   ctx->npoints = n;
+  return 0;
+}
+
+// Checked ingestion (mgb_set_points_checked): the ingestion above with the canonical-encoding bit, then k_check_points
+// over the whole table.  found = {number of invalid points, index of the first, its status byte}.  The context keeps
+// the points only when every one is valid.
+template <class CV>
+int set_points_checked_impl(mgb_ctx* ctx, const uint8_t* xy, const uint8_t* is_zero, size_t n, uint8_t* status, uint32_t* found) {
+  static_assert(PT_NONCANONICAL == MGB_PT_NONCANONICAL && PT_OFF_CURVE == MGB_PT_OFF_CURVE && PT_NOT_IN_SUBGROUP == MGB_PT_NOT_IN_SUBGROUP, "status bits");
+  ENS(ctx, ctx->checks, 8 + n);
+  uint32_t* counters = (uint32_t*)ctx->checks.p;
+  uint8_t* d_status = (uint8_t*)ctx->checks.p + 8;
+  int rc = set_points_impl<CV>(ctx, xy, is_zero, n, d_status);
+  ctx->npoints = 0;                                                 // (set_points_impl stored n)
+  if (rc) return rc;
+  CU(ctx, cudaMemsetAsync(counters, 0, 8, ctx->stream));
+  k_check_points<CV><<<cdiv(n, 128), 128, 0, ctx->stream>>>((uint32_t)n, (const uint32_t*)ctx->table.p, d_status, counters);
+  CU(ctx, cudaGetLastError());
+  CU(ctx, cudaMemcpyAsync(found, counters, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  if (status) CU(ctx, cudaMemcpyAsync(status, d_status, n, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(ctx, cudaStreamSynchronize(ctx->stream));
+  found[1] = ~found[1];                                             // k_check_points keeps the complement of the index
+  found[2] = 0;
+  if (found[0]) {
+    uint8_t why = 0;
+    CU(ctx, cudaMemcpyAsync(&why, d_status + found[1], 1, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    found[2] = why;
+  } else {
+    ctx->npoints = n;
+  }
   return 0;
 }
 
@@ -807,6 +842,23 @@ int msm_common(mgb_ctx* ctx, const void* scalars, bool dev, size_t n, const mgb_
   DISPATCH(ctx, msm_impl, ctx, scalars, dev, n, opts, out_xy, out_is_zero, tm);
 }
 
+// argument checks + checked ingestion of one context (found: see set_points_checked_impl)
+int set_points_checked_ctx(mgb_ctx* ctx, const uint8_t* xy_le, const uint8_t* is_zero, size_t n, uint8_t* status, uint32_t* found) {
+  found[0] = found[1] = found[2] = 0;
+  if (n > ctx->max_points) return fail(ctx, MGB_E_INVALID, "mgb_set_points_checked: n exceeds max_points");
+  CU(ctx, cudaSetDevice(ctx->device));
+  ctx->npoints = 0;
+  if (n == 0) return 0;
+  DISPATCH(ctx, set_points_checked_impl, ctx, xy_le, is_zero, n, status, found);
+}
+
+std::string invalid_points_message(uint64_t count, uint64_t first, uint32_t why) {
+  const char* reason = (why & MGB_PT_NONCANONICAL) ? "non-canonical encoding (x or y >= p)"
+                       : (why & MGB_PT_OFF_CURVE)  ? "not on the curve"
+                                                   : "not in the prime-order subgroup";
+  return std::to_string(count) + (count == 1 ? " invalid point" : " invalid points") + "; the first is point " + std::to_string(first) + ": " + reason;
+}
+
 int multi_fail(mgb_multi* m, int code, const std::string& msg) {
   if (m) m->err = msg;
   g_last_error = msg;
@@ -879,6 +931,16 @@ int mgb_set_points(mgb_ctx* ctx, const uint8_t* xy_le, const uint8_t* is_zero, s
   CU(ctx, cudaSetDevice(ctx->device));
   if (n == 0) { ctx->npoints = 0; return 0; }
   DISPATCH(ctx, set_points_impl, ctx, xy_le, is_zero, n);
+}
+
+int mgb_set_points_checked(mgb_ctx* ctx, const uint8_t* xy_le, const uint8_t* is_zero, size_t n, uint8_t* status, uint64_t* n_invalid) {
+  if (!ctx || (!xy_le && n)) return fail(ctx, MGB_E_INVALID, "mgb_set_points_checked: NULL argument");
+  uint32_t found[3];
+  int rc = set_points_checked_ctx(ctx, xy_le, is_zero, n, status, found);
+  if (rc) return rc;
+  if (n_invalid) *n_invalid = found[0];
+  if (found[0]) return fail(ctx, MGB_E_INVALID, invalid_points_message(found[0], found[1], found[2]));
+  return 0;
 }
 
 int mgb_random_points(mgb_ctx* ctx, uint64_t seed, size_t n) {
@@ -1035,6 +1097,29 @@ int mgb_multi_set_points(mgb_multi* m, const uint8_t* xy_le, const uint8_t* is_z
   });
 }
 
+int mgb_multi_set_points_checked(mgb_multi* m, const uint8_t* xy_le, const uint8_t* is_zero, size_t n, uint8_t* status, uint64_t* n_invalid) {
+  if (!m || (!xy_le && n)) return multi_fail(m, MGB_E_INVALID, "mgb_multi_set_points_checked: NULL argument");
+  multi_shards(m, n);
+  const size_t G = m->ctxs.size(), pb = point_bytes(m->ctxs[0]->curve);
+  std::vector<uint32_t> found(3 * G, 0);
+  int rc = multi_each(m, [&](size_t g) {
+    return set_points_checked_ctx(m->ctxs[g], xy_le + m->lo[g] * pb, is_zero ? is_zero + m->lo[g] : nullptr, m->hi[g] - m->lo[g],
+                                  status ? status + m->lo[g] : nullptr, &found[3 * g]);
+  });
+  uint64_t count = 0, first = 0;
+  uint32_t why = 0;
+  for (size_t g = G; g-- > 0;)                                      // the lowest shard with an invalid point names the first
+    if (found[3 * g]) { count += found[3 * g]; first = m->lo[g] + found[3 * g + 1]; why = found[3 * g + 2]; }
+  if (rc || count) {                                                // no device keeps its shard
+    for (mgb_ctx* c : m->ctxs) c->npoints = 0;
+    m->npoints = 0;
+  }
+  if (rc) return rc;
+  if (n_invalid) *n_invalid = count;
+  if (count) return multi_fail(m, MGB_E_INVALID, invalid_points_message(count, first, why));
+  return 0;
+}
+
 int mgb_multi_random_points(mgb_multi* m, uint64_t seed, size_t n) {
   if (!m) return multi_fail(m, MGB_E_INVALID, "mgb_multi_random_points: NULL argument");
   multi_shards(m, n);
@@ -1084,7 +1169,7 @@ void mgb_destroy(mgb_ctx* ctx) {
   if (ctx->comm) { if (NcclApi* api = nccl_api()) api->CommDestroy(ctx->comm); ctx->comm = nullptr; }
   if (ctx->gathered.p) cudaFree(ctx->gathered.p);
   DevBuf* bufs[] = {&ctx->table, &ctx->scalars, &ctx->ent_bucket, &ctx->ent_rank, &ctx->counts, &ctx->offs, &ctx->offcnt, &ctx->tile_sums, &ctx->pairs, &ctx->pairs2, &ctx->V, &ctx->W, &ctx->recs, &ctx->lifes, &ctx->prebuf, &ctx->bsum, &ctx->redU[0], &ctx->redU[1], &ctx->redW[0], &ctx->redW[1], &ctx->misc,
-                    &ctx->acc_out, &ctx->out_xy, &ctx->stage};
+                    &ctx->acc_out, &ctx->out_xy, &ctx->stage, &ctx->checks};
   for (DevBuf* b : bufs) if (b->p) cudaFree(b->p);
   for (auto& q : ctx->pf) { if (q.buf.p) cudaFree(q.buf.p); if (q.ev) cudaEventDestroy(q.ev); }
   if (ctx->pf_stream) cudaStreamDestroy(ctx->pf_stream);

@@ -59,8 +59,9 @@ class ShardedMsm:
         if self.world > 1:
             self.engine.comm_init(exchange_comm_id(self.rank, local_device), self.rank, self.world)
 
-    def set_points(self, xy_bytes_shard, is_zero=None):
-        return self.engine.set_points(xy_bytes_shard, is_zero)
+    def set_points(self, xy_bytes_shard, is_zero=None, check=False):
+        """check=True: this rank's shard is checked on its device (MsmEngine.set_points); indices are shard-local."""
+        return self.engine.set_points(xy_bytes_shard, is_zero, check=check)
 
     def random_points(self, n_local: int, seed: int):
         """Known-dlog points; rank r uses seed + r so the global set is the union of the shards."""

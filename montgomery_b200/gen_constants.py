@@ -46,6 +46,39 @@ def field_struct(name, p, n, fid):
     return out
 
 
+def subgroup_consts(z_abs, beta_squared):
+    """Membership test of G1 in mgb_set_points_checked: sigma'(P) + P == [z^2] P, sigma'(x, y) = (beta' x, y) with beta'
+    the cube root of unity whose eigenvalue on G1 is z^2 - 1 (DESIGN.md, checked point ingestion).  z^2 is one binary
+    chain of 127 or 128 bits.  Z2 = 0: the cofactor is 1 and every point on the curve is in the group."""
+    z2 = z_abs * z_abs
+    if z_abs:
+        out = "  // z^2 of the BLS12 parameter (|z| = 0x%x) in two 64-bit halves, Z2_TOP = its top bit\n" % z_abs
+    else:
+        out = "  // cofactor 1: no subgroup chain\n"
+    out += "  static constexpr uint64_t Z2_HI = 0x%016xull, Z2_LO = 0x%016xull;\n" % (z2 >> 64, z2 & (2**64 - 1))
+    out += "  static constexpr int Z2_TOP = %d;\n" % (z2.bit_length() - 1)
+    out += "  static constexpr bool SIGMA_BETA_SQUARED = %s;  // sigma'(x, y) = (beta^2 x, y) instead of (beta x, y)\n" % ("true" if beta_squared else "false")
+    return out
+
+
+def naf_masks(k):
+    """non-adjacent form of k as two bit masks (positions of the +1 and of the -1 digits)"""
+    pos = neg = 0
+    i = 0
+    while k:
+        if k & 1:
+            d = 2 - (k & 3)
+            k -= d
+            if d > 0:
+                pos |= 1 << i
+            else:
+                neg |= 1 << i
+        k >>= 1
+        i += 1
+    assert pos - neg > 0 and pos & neg == 0 and pos & (pos >> 1) == 0
+    return pos, neg
+
+
 def egcd_stop_early(l, p):
     r0, r1, t0, t1 = p, l, 0, 1
     while r1 * r1 > p:
@@ -132,24 +165,35 @@ def main():
     out += carr("b3", mont(3 * 1, p377, 12), 12)
     out += carr("gx", mont(g377[0], p377, 12), 12)
     out += carr("gy", mont(g377[1], p377, 12), 12)
-    out += "  static constexpr int SCALAR_BITS = 253;\n};\n\n"
+    out += "  static constexpr int SCALAR_BITS = 253;\n"
+    out += subgroup_consts(0x8508C00000000001, beta_squared=True)      # beta^2: eigenvalue z^2 - 1 (the GLV lambda is the other root)
+    out += "};\n\n"
     out += "struct PallasConsts {\n"
     out += carr("beta", mont(betapal, ppal, 8), 8)
     out += carr("b3", mont(3 * 5, ppal, 8), 8)
     out += carr("gx", mont(gpal[0], ppal, 8), 8)
     out += carr("gy", mont(gpal[1], ppal, 8), 8)
-    out += "  static constexpr int SCALAR_BITS = 255;\n};\n\n"
+    out += "  static constexpr int SCALAR_BITS = 255;\n"
+    out += subgroup_consts(0, beta_squared=False)                       # cofactor 1
+    out += "};\n\n"
     out += "struct Bls12381Consts {\n"
     out += carr("beta", mont(beta381, p381, 12), 12)
     out += carr("b3", mont(3 * 4, p381, 12), 12)
     out += carr("gx", mont(g381[0], p381, 12), 12)
     out += carr("gy", mont(g381[1], p381, 12), 12)
-    out += "  static constexpr int SCALAR_BITS = 255;\n};\n\n"
+    out += "  static constexpr int SCALAR_BITS = 255;\n"
+    out += subgroup_consts(0xD201000000010000, beta_squared=False)     # beta: eigenvalue z^2 - 1 = the GLV lambda
+    out += "};\n\n"
     out += "struct Ed377Consts {\n"
     out += carr("k", mont(2 * 3021, q377, 8), 8)     # k = 2d
     out += carr("gx", mont(ged[0], q377, 8), 8)
     out += carr("gy", mont(ged[1], q377, 8), 8)
     out += carr("q", qed, 8)
+    pos, neg = naf_masks(qed)
+    out += "  // [q]P == O test of mgb_set_points_checked: q in non-adjacent form, digit i = +1 / -1 where bit i of naf_pos / naf_neg is set\n"
+    out += carr("naf_pos", pos, 8)
+    out += carr("naf_neg", neg, 8)
+    out += "  static constexpr int NAF_TOP = %d;  // the top digit, +1\n" % (pos.bit_length() - 1)
     out += "  static constexpr int SCALAR_BITS = 251;\n};\n\n"
     s, info377 = glv_struct("Glv377", q377, lam377)
     out += s
